@@ -10,6 +10,7 @@ reference architectures.
     python bench.py --impl reference ...      # the reference networks on the host CPU cores
     python bench.py --impl torch-cuda ...     # GPU STAND-IN for the reference's CUDA build (not the reference arm):
                                               # the oracle port of its networks on CUDA under fp16 autocast
+    python bench.py --gpus 1 --steps 10 --warmup 3 --dump-outputs DIR   # + what the last timed step returned, as .npy
 
 A step = one pass of the hot path over one frame.  `value` = hypotheses / step time with the frame,
 mesh and weights resident in HBM (device-timed with CUDA events, max over ranks); `e2e` = the same
@@ -185,6 +186,14 @@ def cpu_nets_rate(budget_s=20.0):
                          f"{t_ref * 1e3:.1f} ms/hyp-iter refine, {t_sc * 1e3:.1f} ms/hyp score; extrapolated to {N_ITER} iters + 1 score; raster/warp not included")
 
 
+def dump_outputs(out_dir, poses, scores, best):
+    """The arrays ShardedRegister.run hands its caller, as float32 / float64 .npy files (12 KB in all at 252 hypotheses)."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "poses.npy"), poses.detach().float().cpu().numpy())      # (252, 4, 4) refined poses
+    np.save(os.path.join(out_dir, "scores.npy"), scores.detach().float().cpu().numpy())    # (252,) scorer logits + 100
+    np.save(os.path.join(out_dir, "best.npy"), np.asarray(int(best.item()), dtype=np.float64))  # index of the selected pose
+
+
 _REAL_STDOUT = None
 
 
@@ -340,7 +349,14 @@ def main():
     ap.add_argument("--no-standin", action="store_true", help="skip the torch-cuda stand-in / parity legs of the native line")
     ap.add_argument("--no-track", action="store_true", help="skip the track_one (BASELINE.json configs[2]) leg")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (refined poses, scores, best index) to DIR/<name>.npy; "
+                         "the inputs are seeded, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs applies to the native path only")
     args.warmup = max(args.warmup, 3) if args.impl == "native" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -444,6 +460,8 @@ def main():
         barrier()
     ms = e0.elapsed_time(e1) / args.steps
     launches = (_lib.launch_count() - launches0) // args.steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, poses_out, scores, best)
     if world > 1:
         t = torch.tensor([ms], device="cuda")
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

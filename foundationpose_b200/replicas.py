@@ -46,14 +46,20 @@ class _Worker(threading.Thread):
             self.est.reset_object(model_pts, model_normals, symmetry_tfs=symmetry_tfs, mesh=mesh)
 
     def run(self):
-        if self.make_estimator is None or torch.cuda.is_available():
-            torch.cuda.set_device(self.device)
+        # a custom estimator's device id may be a label only (the host-side test double): select it only if it exists
+        try:
+            if self.make_estimator is None or self.device < torch.cuda.device_count():
+                torch.cuda.set_device(self.device)
+        except Exception as ex:  # no such device: every job fails with this, instead of the caller waiting forever
+            self.error = ex
         while True:
             job = self.jobs.get()
             if job is None:
                 return
             kind, payload, done = job
             try:
+                if self.error is not None:
+                    raise self.error
                 if kind == "reset":
                     model_pts, model_normals, mesh, symmetry_tfs = payload
                     if self.est is None:

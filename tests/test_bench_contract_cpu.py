@@ -21,3 +21,11 @@ def test_reference_arm_prints_the_contract_line():
     cb = d["cpu_baseline"]
     assert cb["kind"] == "port" and cb["cores"] >= 1 and cb["value"] == d["value"] and cb["unit"] == "hyp/s" and "sample" in cb
     assert d["e2e"] == {"value": d["value"], "unit": "hyp/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
+
+
+def test_bench_rejects_zero_steps_and_dumps_of_other_arms(tmp_path):
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path)]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True, timeout=300, cwd=ROOT)
+        assert out.returncode == 2 and "error:" in out.stderr, (extra, out.stderr[-2000:])
+        assert out.stdout == ""
+    assert not os.listdir(tmp_path)

@@ -47,24 +47,15 @@ def test_cluster_poses_matches_the_reference_cpp(golden):
 
 
 def test_cluster_poses_against_the_compiled_reference_function(golden):
-    """The same, live against oracle/_ref/libcluster_ref.so (built by __graft_entry__.build() where /root/reference
-    exists; it travels to the GPU box with the snapshot) on random pose sets the fixture does not hold."""
+    """The same, on random pose sets: what the compiled reference function (oracle/_ref/libcluster_ref.so, built by
+    oracle/build_ref.py) kept of each set, stored as indices into it by tools/make_golden_cluster.py."""
     from foundationpose_b200 import hypotheses as hy
-    from oracle import build_ref
 
-    ref = build_ref.load()
-    if ref is None:
-        pytest.skip("oracle/_ref/libcluster_ref.so not built (no reference tree)")
-    gen, g = golden
-    from scipy.spatial.transform import Rotation
-
-    rng = np.random.default_rng(3)
+    gen, _ = golden
+    g = np.load(os.path.join(ROOT, "tests", "golden", "cluster_random_golden.npz"))
     for trial in range(4):
-        n = 150
-        poses = np.tile(np.eye(4, dtype=np.float32), (n, 1, 1))
-        poses[:, :3, :3] = Rotation.random(n, random_state=trial).as_matrix()
-        poses[:, :3, 3] = rng.normal(0, 0.02, (n, 3))
+        poses = g[f"poses.{trial}"]
         for name, syms in gen.symmetry_sets().items():
             a = hy.cluster_poses(25 + 5 * trial, 0.03, poses, syms)
-            b = ref(25 + 5 * trial, 0.03, poses, syms)
+            b = poses[g[f"kept.{trial}.{name}"]]
             assert a.shape == b.shape and np.array_equal(a, b), (trial, name, a.shape, b.shape)

@@ -1,6 +1,6 @@
 """CPU: the drop-in module tree (foundationpose_b200/dropin) resolves every name the reference's UNMODIFIED
 run_demo.py uses, the trimesh / imageio stand-ins round-trip the demo-scene files, and the reader parses them."""
-import ast
+import json
 import os
 import subprocess
 import sys
@@ -9,7 +9,6 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 DROPIN = os.path.join(ROOT, "foundationpose_b200", "dropin")
-REF_DEMO = "/root/reference/run_demo.py"
 
 
 def _env():
@@ -18,22 +17,19 @@ def _env():
     return env
 
 
-@pytest.mark.skipif(not os.path.exists(REF_DEMO), reason="reference tree not present (GPU box)")
+def _driver_names(script):
+    """Import statements, unqualified names and first-level attributes of one of the reference's drivers, read from the
+    driver with `ast` by tools/make_golden_drivers.py --names."""
+    with open(os.path.join(ROOT, "tests", "golden", "driver_names.json")) as fh:
+        d = json.load(fh)[script]
+    return d["imports"], d["names"], [tuple(a) for a in d["attrs"]]
+
+
 def test_every_name_run_demo_uses_resolves():
     """Static check against the reference's own driver: all unqualified names and first-level attributes
     (`trimesh.load`, `dr.RasterizeCudaContext`, `np.stack`, ...) exist after its two star-imports."""
-    import builtins
-
-    tree = ast.parse(open(REF_DEMO).read())
-    assigned, used, attrs = set(), set(), set()
-    for node in ast.walk(tree):
-        if isinstance(node, ast.Name):
-            (assigned if isinstance(node.ctx, ast.Store) else used).add(node.id)
-        elif isinstance(node, ast.Attribute) and isinstance(node.value, ast.Name):
-            attrs.add((node.value.id, node.attr))
-    need = sorted(n for n in used - assigned - set(dir(builtins)) if n != "__file__")
+    _, need, mod_attrs = _driver_names("run_demo.py")
     assert {"trimesh", "dr", "np", "cv2", "imageio", "logging", "set_seed", "YcbineoatReader", "FoundationPose"} <= set(need)
-    mod_attrs = sorted((m, a) for (m, a) in attrs if m in need and m not in ("args", "parser", "o3d"))
     code = ("from estimater import *\nfrom datareader import *\nimport argparse\n"
             f"missing = [n for n in {need!r} if n not in globals()]\n"
             f"missing += [f'{{m}}.{{a}}' for (m, a) in {mod_attrs!r} if m in globals() and not hasattr(globals()[m], a)]\n"
@@ -84,24 +80,8 @@ print('OK')
 def test_every_name_the_dataset_drivers_use_resolves(script):
     """Same static check for the reference's dataset drivers (SURVEY.md §8f N3): replay the script's own import
     statements on top of the drop-in tree, then every unqualified name / first-level attribute must exist."""
-    import builtins
-
-    path = "/root/reference/" + script
-    if not os.path.exists(path):
-        pytest.skip("reference tree not present (GPU box)")
-    tree = ast.parse(open(path).read())
-    imports = [ast.unparse(n) for n in tree.body if isinstance(n, (ast.Import, ast.ImportFrom))]
-    assigned, used, attrs = set(), set(), set()
-    for node in ast.walk(tree):
-        if isinstance(node, ast.Name):
-            (assigned if isinstance(node.ctx, ast.Store) else used).add(node.id)
-        elif isinstance(node, ast.Attribute) and isinstance(node.value, ast.Name):
-            attrs.add((node.value.id, node.attr))
-        elif isinstance(node, (ast.FunctionDef, ast.arg)):
-            assigned.add(node.name if isinstance(node, ast.FunctionDef) else node.arg)
-    need = sorted(n for n in used - assigned - set(dir(builtins)) if n != "__file__")
+    imports, need, mod_attrs = _driver_names(script)
     assert {"wp", "NestDict", "make_yaml_dumpable", "dr", "trimesh", "FoundationPose", "set_seed", "argparse"} <= set(need)
-    mod_attrs = sorted((m, a) for (m, a) in attrs if m in need and m not in ("opt", "parser", "o3d", "reader", "reader_tmp", "est"))
     code = ("\n".join(imports) + "\n"
             f"missing = [n for n in {need!r} if n not in globals()]\n"
             f"missing += [f'{{m}}.{{a}}' for (m, a) in {mod_attrs!r} if m in globals() and not hasattr(globals()[m], a)]\n"

@@ -336,3 +336,18 @@ def test_unsupported_config_raises():
         estimater._load_cfg_and_weights("x", "score", sd, {"input_resize": [128, 128]})
     cfg, _ = estimater._load_cfg_and_weights("x", "score", sd, {"crop_ratio": 1.1})
     assert cfg["crop_ratio"] == 1.1 and cfg["rot_rep"] == weights.DEFAULT_CFG["rot_rep"]
+
+
+def test_replica_pool_surfaces_a_missing_device():
+    """A replica whose GPU does not exist fails every call with the reason instead of leaving the caller waiting."""
+    from foundationpose_b200.replicas import ReplicaPool
+
+    pool = ReplicaPool([4096])
+    try:
+        with pytest.raises(RuntimeError):
+            pool.reset_object(None, None)
+        with pytest.raises(RuntimeError):
+            pool.register_many([(None, 0, None, None)])
+    finally:
+        pool.close()
+    assert not any(w.is_alive() for w in pool.workers)

@@ -8,10 +8,11 @@
     Two third-party pieces are substituted: `trimesh.creation.icosphere` (trimesh is absent; this repository's icosphere
     is used — its VERTEX ORDER is therefore not pinned, SURVEY.md §8c) and `transformations.euler_matrix` (scipy).
 
-    python tools/make_golden_cluster.py     # needs /root/reference; writes tests/golden/cluster_golden.npz
+    python tools/make_golden_cluster.py     # needs the reference tree (FPOSE_REFERENCE); writes
+                                            # tests/golden/cluster_golden.npz and cluster_random_golden.npz
 
 tests/test_cluster_golden_cpu.py holds foundationpose_b200.hypotheses (cluster_poses, sample_views_icosphere,
-make_rotation_grid) to these vectors, and to the compiled reference function directly when oracle/_ref/ holds it.
+make_rotation_grid) to these vectors.
 """
 import logging
 import os
@@ -77,6 +78,26 @@ def main():
         for ang in (10, 61):
             out[f"cluster.{name}.{ang}"] = cluster(ang, 99999, grid, syms)
     out["cluster.moved.half_z"] = cluster(30, 0.01, moved, symmetry_sets()["half_z"])
+    # random pose sets with translations spread over the distance threshold, one angle threshold per set; what the
+    # reference keeps is stored as indices into the set (it returns a subset of its input poses, unchanged)
+    from scipy.spatial.transform import Rotation
+
+    rng = np.random.default_rng(3)
+    rand = {}
+    for trial in range(4):
+        n = 150
+        poses = np.tile(np.eye(4, dtype=np.float32), (n, 1, 1))
+        poses[:, :3, :3] = Rotation.random(n, random_state=trial).as_matrix()
+        poses[:, :3, 3] = rng.normal(0, 0.02, (n, 3))
+        rand[f"poses.{trial}"] = poses
+        for name, syms in symmetry_sets().items():
+            kept = cluster(25 + 5 * trial, 0.03, poses, syms)
+            idx = [int(np.flatnonzero((poses == k).all(axis=(1, 2)))[0]) for k in kept]
+            assert np.array_equal(poses[idx], kept)
+            rand[f"kept.{trial}.{name}"] = np.array(idx, dtype=np.int16)
+    dst = os.path.join(ROOT, "tests", "golden", "cluster_random_golden.npz")
+    np.savez_compressed(dst, **rand)
+    print(f"wrote {dst}: {len(rand)} entries, {os.path.getsize(dst) / 1024:.0f} KiB")
     dst = os.path.join(ROOT, "tests", "golden", "cluster_golden.npz")
     np.savez_compressed(dst, **out)
     print(f"wrote {dst}: {len(out)} entries, {os.path.getsize(dst) / 1024:.0f} KiB")
