@@ -116,6 +116,46 @@ int fp_op_attention(const void* qkv, void* out, int B, int impl, void* stream) {
   return fp::attn_tc_launch(ap, st);
 }
 
+int fp_op_attention_grouped(const void* qkv, void* out, int B, int n_groups, void* stream) {
+  if (!qkv || !out || B < 0 || (n_groups != 1 && n_groups != 2)) {
+    fp::set_last_error("fp_op_attention_grouped: null argument, B < 0 or n_groups not 1 / 2");
+    return -1;
+  }
+  // the AttnParams of run_score_feats (n_groups = 1) and run_refine_heads (n_groups = 2) in fp_api.cu
+  fp::AttnParams ap;
+  ap.qkv = reinterpret_cast<const __half*>(qkv);
+  ap.ld = 1536 * n_groups;
+  ap.q_off = 0;
+  ap.k_off = 512;
+  ap.v_off = 1024;
+  ap.group_col_stride = n_groups == 2 ? 1536 : 0;
+  ap.n_groups = n_groups;
+  ap.out = reinterpret_cast<__half*>(out);
+  ap.ld_out = 512;
+  ap.out_group_stride = n_groups == 2 ? (size_t)B * 400 * 512 : 0;
+  ap.B = B;
+  ap.T = 400;
+  ap.n_heads = 4;
+  ap.scale = 0.08838834764831845f;
+  return fp::attn_core_launch(ap, reinterpret_cast<cudaStream_t>(stream));
+}
+
+int fp_op_gemm_last_plan(int* out, int n) {
+  if (!out || n < 0) {
+    fp::set_last_error("fp_op_gemm_last_plan: null output");
+    return -1;
+  }
+  fp::GemmPlan pl;
+  if (!fp::last_plan(&pl)) {
+    fp::set_last_error("fp_op_gemm_last_plan: no GEMM launch on this thread yet");
+    return -1;
+  }
+  const int v[FP_GEMM_PLAN_FIELDS] = {pl.kernel, pl.bn,   pl.cg, pl.slabs, pl.patch,   pl.grid,
+                                      pl.work_tiles, pl.bw, pl.bh, pl.bimg, pl.m_tiles, pl.n_tiles};
+  for (int i = 0; i < n && i < FP_GEMM_PLAN_FIELDS; ++i) out[i] = v[i];
+  return 0;
+}
+
 int fp_op_gemm_layer(const fp_gemm_layer_t* l, void* stream) {
   if (!l) {
     fp::set_last_error("fp_op_gemm_layer: null layer");

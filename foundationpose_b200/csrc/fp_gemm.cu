@@ -108,6 +108,17 @@ void set_last_error(const char* fmt, ...) {
 }
 const char* get_last_error() { return t_last_error; }
 
+static thread_local GemmPlan t_plan;
+static thread_local bool t_plan_set = false;
+void note_plan(const GemmPlan& plan) {
+  t_plan = plan;
+  t_plan_set = true;
+}
+bool last_plan(GemmPlan* plan) {
+  if (t_plan_set) *plan = t_plan;
+  return t_plan_set;
+}
+
 static thread_local int t_pdl_skip = 0;
 void pdl_skip_next() { t_pdl_skip = 1; }
 
@@ -1210,6 +1221,8 @@ static int launch_bn(const CUtensorMap& ma, const CUtensorMap& mb, const CUtenso
   const int total_vt = ((m_tiles + CG - 1) / CG) * p.n_tiles_n;
   const int slots = g_num_sms / CG;
   const int grid = CG * (total_vt < slots ? total_vt : slots);
+  note_plan({PK_TILE, BN, CG, SLABS, PATCH ? (p.seg_count == 3 ? 2 : 1) : 0, grid, total_vt * CG, p.bw, p.bh, p.bn, m_tiles,
+             p.n_tiles_n});
   prof_mark_begin(0, p.alg_flops, stream);
 #ifdef FP_GEMM_TRACE
   GemmParams pt = p;
@@ -1242,6 +1255,7 @@ static int launch_swap(const CUtensorMap& ma, const CUtensorMap& mw, const CUten
   const int m_tiles = p.tiles_w * p.tiles_h * p.tiles_n;
   const int total_vt = ((m_tiles + 1) / 2) * (p.Cout / 128);
   const int grid = total_vt < g_num_sms ? total_vt : g_num_sms;
+  note_plan({PK_SWAP, 128, 1, 0, 0, grid, total_vt, p.bw, p.bh, p.bn, m_tiles, p.Cout / 128});
   prof_mark_begin(0, p.alg_flops, stream);
   FP_CUDA_OK(launch_pdl(gemm_swap_kernel, dim3(grid), dim3(kTileThreads), kSwapSmem, stream, 1, ma, mw, mo, mr, p));
   prof_mark_end(stream);
@@ -1259,8 +1273,10 @@ static int launch_swap_patch(const CUtensorMap& ma, const CUtensorMap& mw, const
   }
   const int sms = num_sms();
   FP_REQUIRE(sms > 0, "no CUDA device");
-  const int total_vt = p.tiles_w * p.tiles_h * p.tiles_n * (p.Cout / 128);
+  const int m_tiles = p.tiles_w * p.tiles_h * p.tiles_n;
+  const int total_vt = m_tiles * (p.Cout / 128);
   const int grid = total_vt < sms ? total_vt : sms;
+  note_plan({PK_SWAP_PATCH, 128, 1, 0, 1, grid, total_vt, p.bw, p.bh, p.bn, m_tiles, p.Cout / 128});
   prof_mark_begin(0, p.alg_flops, stream);
   FP_CUDA_OK(launch_pdl(gemm_swap_patch_kernel, dim3(grid), dim3(kTileThreads), kSwapPatchSmem, stream, 1, ma, mw, mo, mr, p));
   prof_mark_end(stream);

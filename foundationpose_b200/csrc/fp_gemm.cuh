@@ -40,6 +40,20 @@ struct GemmLayer {
 // Enqueue one layer on `stream`.  Returns 0 or a negative error code (fp_last_error() has text).
 int gemm_layer_launch(const GemmLayer& L, cudaStream_t stream);
 
+// What a launch chose (fp_op_gemm_last_plan, include/fpose.h): kept per host thread, a few stores per launch.
+enum PlanKernel : int { PK_TILE = 0, PK_SWAP = 1, PK_SWAP_PATCH = 2, PK_STEM = 3 };
+struct GemmPlan {
+  int kernel;        // PlanKernel
+  int bn, cg, slabs; // output channels per tile, CTAs per MMA, epilogue staging slabs (tile kernel only, else 0)
+  int patch;         // 0: one TMA box per tap, 1: one halo'd patch per channel chunk, 2: column-shifted copies
+  int grid;          // CTAs launched
+  int work_tiles;    // loop iterations summed over the grid: a CTA runs ceil(work_tiles / grid) of them
+  int bw, bh, bimg;  // one M tile = bw x bh pixels of bimg images (LINEAR: bw = 128 rows)
+  int m_tiles, n_tiles;  // M tiles of the launch, channel blocks of `bn` (swap kernels: 128) per M tile
+};
+void note_plan(const GemmPlan& plan);
+bool last_plan(GemmPlan* plan);  // false before this thread's first launch
+
 
 // Optional per-launch device timing (CUDA events on the launching stream) of the two kernels the
 // roofline is reported for: kind 0 = gemm_tile_kernel (work = algorithmic FLOPs), kind 1 = crop_kernel

@@ -281,6 +281,7 @@ int stem_conv_launch(const GemmLayer& L, cudaStream_t stream) {
   const int sms = num_sms();
   FP_REQUIRE(sms > 0, "no CUDA device");
   const int grid = p.total_tiles < sms ? p.total_tiles : sms;
+  note_plan({PK_STEM, 64, 1, 0, 0, grid, p.total_tiles, kTileW, kTileH, 1, p.total_tiles, 1});
   prof_mark_begin(0, 2.0 * (double)L.n_img * Ho * Wo * 64.0 * (7.0 * 7.0 * 6.0), stream);
   FP_CUDA_OK(launch_pdl(stem_conv_kernel, dim3(grid), dim3(kThreadsStem), kStemSmem, stream, 1, mi, mo,
                         reinterpret_cast<const __half*>(L.w), p));

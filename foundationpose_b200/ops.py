@@ -57,3 +57,37 @@ def attention(qkv, impl=1):
     out = torch.empty(qkv.shape[0], 512, dtype=torch.float16, device=qkv.device)
     _lib.check(lib.fp_op_attention(_ptr(qkv), _ptr(out), B, impl, _stream()), "fp_op_attention")
     return out
+
+
+lib.fp_op_attention_grouped.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]
+lib.fp_op_attention_grouped.restype = C.c_int
+
+
+def attention_grouped(qkv, n_groups):
+    """The product's attention launch: n_groups = 1 (scorer) qkv fp16 [B*400, 1536] -> [B*400, 512];
+    n_groups = 2 (refiner, both heads) qkv fp16 [B*400, 3072] -> [2, B*400, 512]."""
+    _require_cuda(qkv)
+    assert n_groups in (1, 2)
+    assert qkv.dtype == torch.float16 and qkv.shape[1] == 1536 * n_groups and qkv.shape[0] % 400 == 0
+    assert qkv.is_contiguous()
+    B = qkv.shape[0] // 400
+    out = torch.empty(n_groups, qkv.shape[0], 512, dtype=torch.float16, device=qkv.device)
+    _lib.check(lib.fp_op_attention_grouped(_ptr(qkv), _ptr(out), B, n_groups, _stream()), "fp_op_attention_grouped")
+    return out if n_groups == 2 else out[0]
+
+
+GEMM_PLAN_FIELDS = ("kernel", "bn", "cg", "slabs", "patch", "grid", "work_tiles", "bw", "bh", "bimg", "m_tiles",
+                    "n_tiles")
+GEMM_KERNELS = ("tile", "swap", "swap_patch", "stem")
+lib.fp_op_gemm_last_plan.argtypes = [C.POINTER(C.c_int), C.c_int]
+lib.fp_op_gemm_last_plan.restype = C.c_int
+
+
+def gemm_last_plan():
+    """What the last GEMM launch on this thread chose (include/fpose.h fp_op_gemm_last_plan), as a dict; `kernel` is
+    one of GEMM_KERNELS."""
+    buf = (C.c_int * len(GEMM_PLAN_FIELDS))()
+    _lib.check(lib.fp_op_gemm_last_plan(buf, len(GEMM_PLAN_FIELDS)), "fp_op_gemm_last_plan")
+    plan = dict(zip(GEMM_PLAN_FIELDS, list(buf)))
+    plan["kernel"] = GEMM_KERNELS[plan["kernel"]]
+    return plan

@@ -75,6 +75,22 @@ int fp_op_gemm_layer(const fp_gemm_layer_t* layer, void* stream);
  * qkv fp16 [B*400][1536] (q | k | v, 4 heads of 128 each), out fp16 [B*400][512].
  * `impl` is ignored (kept for ABI stability): there is one implementation, the tcgen05 kernel. */
 int fp_op_attention(const void* qkv, void* out, int B, int impl, void* stream);
+/* The same attention in the two layouts the product runs: n_groups = 1 is the scorer's (score_network.py:53;
+ * qkv [B*400][1536], out [B*400][512]), n_groups = 2 the refiner's two heads in one launch (refine_network.py:56-70;
+ * qkv [B*400][3072] = head 0's q | k | v then head 1's, out [2][B*400][512]). */
+int fp_op_attention_grouped(const void* qkv, void* out, int B, int n_groups, void* stream);
+
+/* What the last fp_op_gemm_layer / product GEMM launch on the calling thread chose (host-side record, no
+ * synchronisation).  Writes min(n, FP_GEMM_PLAN_FIELDS) ints:
+ *   [0] kernel: 0 = gemm_tile_kernel, 1 = gemm_swap_kernel, 2 = gemm_swap_patch_kernel, 3 = stem_conv_kernel
+ *   [1] output channels per tile  [2] CTAs per MMA (cta_group)  [3] epilogue staging slabs (tile kernel, else 0)
+ *   [4] patch mode: 0 = one TMA box per filter tap, 1 = one halo'd patch per channel chunk, 2 = column-shifted copies
+ *   [5] grid  [6] work tiles: loop iterations summed over the grid (a CTA runs ceil([6] / [5]) of them)
+ *   [7..9] one M tile = [7] x [8] pixels (columns x rows) of [9] images (LINEAR: [7] = 128 rows)
+ *   [10] M tiles  [11] channel blocks per M tile
+ * Returns -1 if this thread has launched no GEMM yet.  Layers that produce nothing (0 images) leave it unchanged. */
+#define FP_GEMM_PLAN_FIELDS 12
+int fp_op_gemm_last_plan(int* out, int n);
 
 
 /* ------------------------------------------------------------------------------------------ */
